@@ -15,9 +15,12 @@ value = whole-job frames/s with inputs resident in HBM; e2e = the same step thro
 in pinned HOST memory (H2D inside the timed region) and the compact detections copied back (D2H inside the timed region).
 Both arms print the same `config` dict (same workload, same stages: pre-process + decode + NMS).
 
-Timing: W warm-up steps, then blocks of EXACTLY K steps each bracketed by CUDA events (barrier + synchronize on both sides);
-as many blocks as it takes to cover >= 0.35 s, so that the 100 ms clock sampler has samples INSIDE the timed windows;
-ms_per_step = mean block time / K (max over ranks per block).  Prints ONE JSON line on rank 0.
+Timing: W warm-up steps, then ONE block of exactly K steps bracketed by CUDA events (barrier + synchronize on both sides);
+ms_per_step = block time / K (max over ranks).  The 100 ms clock sampler only has samples inside the timed window when it
+lasts long enough: pick K accordingly.  Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR writes what the timed path computed in its last step (see dump_outputs), so that two builds can be
+compared output for output: the inputs are synthetic and seeded, identical from run to run.
 """
 from __future__ import annotations
 
@@ -25,7 +28,6 @@ import argparse
 import ctypes as C
 import hashlib
 import json
-import math
 import os
 import statistics
 import subprocess
@@ -56,7 +58,7 @@ CONFIGS = {
 }
 ALGO_BYTES_PER_IMAGE = (4 + NC) * sum((NET // s) ** 2 for s in STRIDES) * 4  # 2 822 400 B, SURVEY 8d
 LETTERBOX_BYTES_PER_IMAGE = NET * NET * 3 + 3 * NET * NET * 4                  # 6 144 000 B, SURVEY 8d
-MIN_TIMED_S = 0.35
+DUMP_SAMPLE = 1 << 20   # elements kept of a dumped output larger than this (a fixed, seeded sample)
 
 
 def _env_int(name, default):
@@ -537,7 +539,8 @@ PER_RANK_MS = []   # N > 1: one list per timed block with every rank's own block
 
 
 def timed_blocks(step, K, W, stream, dev, world, dist, flush=None, pre=None, run_many=None):
-    """W warm-up steps, then blocks of exactly K steps; returns (mean ms per block, [(t0, t1) wall windows], n_blocks)."""
+    """W warm-up steps (0 .. W-1), then one block of exactly K steps (W .. W+K-1); returns (ms of the block,
+    [(t0, t1) wall window], 1)."""
     import torch
 
     def block(first):
@@ -579,15 +582,29 @@ def timed_blocks(step, K, W, stream, dev, world, dist, flush=None, pre=None, run
             step(i)
     if flush is not None:
         flush(W - 1)
-    ms0, w0 = block(W)
-    n = max(1, math.ceil(MIN_TIMED_S * 1e3 / max(ms0, 1e-3)))   # same on every rank: ms0 is the max over ranks
-    n = min(n, 4000)
-    res, wins = [ms0], [w0]
-    for b in range(1, n):
-        ms, w = block(W + b * K)
-        res.append(ms)
-        wins.append(w)
-    return sum(res) / len(res), wins, len(res)
+    ms, w = block(W)
+    return ms, [w], 1
+
+
+def dump_outputs(out_dir, arrays: dict) -> None:
+    """arrays: name -> the tensor a caller of the timed path receives, after its last timed step.  Written as
+    out_dir/<name>.npy in float32; a tensor of more than DUMP_SAMPLE elements is reduced to the same DUMP_SAMPLE
+    flat positions on every run (seed 0, ascending).  Compact detection buffers ([B, 1 + max_det * row] with the row count
+    in column 0) are passed with their row width, and their floats past the count, which no caller reads, are zeroed."""
+    import numpy as np
+
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, (t, row) in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if row:
+            a = a.copy()
+            for b in range(a.shape[0]):
+                a[b, 1 + int(a[b, 0]) * row:] = 0
+        if a.size > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(out_dir / f"{name}.npy", np.ascontiguousarray(a, np.float32))
 
 
 def time_kernel_loop(fn, n, stream, dev):
@@ -835,6 +852,9 @@ def run_v8(args, rank, world, local_rank):
         if peer is not None:   # whole groups only
             K, W = max(G, K // G * G), max(G, (W + G - 1) // G * G)
         ms_dev, win_dev, nb_dev = timed_blocks(step_dev, K, W, stream, dev, world, dist, flush_dev, run_many=run_dev)
+        if args.dump_outputs:   # N = 1 without the gather: the last timed step (W + K - 1) wrote its set's pipeline
+            last = pipes_dev[(W + K - 1) % R]
+            dump_outputs(args.dump_outputs, {"detections": (last.fused.out, 7), "net_input": (last.net_input, 0)})
         per_rank_ms = None   # N > 1: every rank's own mean ms per step over the timed blocks (ms_per_step is built from the per-block maxima)
         try:
             if PER_RANK_MS:
@@ -937,7 +957,7 @@ def run_v8(args, rank, world, local_rank):
                 "cuda_graphs": not args.no_graph,
                 "overlap": (f"{G} steps per graph as two concurrent chains: letterbox launches || (scan -> NMS) launches" if G > 1 else
                             ("letterbox || (scan -> NMS) as parallel graph branches" if not args.no_overlap else "serial")),
-                "timed_blocks": {"device": nb_dev, "e2e": nb_e2e, "steps_per_block": K, "min_timed_s": MIN_TIMED_S},
+                "timed_blocks": {"device": nb_dev, "e2e": nb_e2e, "steps_per_block": K},
                 "per_rank_ms_per_step": per_rank_ms,
                 "gpus_during_device_blocks": all_gpus.summary(win_dev) if all_gpus is not None else None,
                 "gather_timeouts": gather_err, "gather_verified": gather_verified,
@@ -1069,6 +1089,13 @@ def run_other(args, local_rank):
         sampler.start()
         time.sleep(0.25)
         ms_dev, win_dev, nb = timed_blocks(step_dev, K, W, stream, dev, 1, None)
+        if args.dump_outputs:   # the last timed step, W + K - 1
+            if name == "rcnn_b8":   # one chain for every input set
+                dump_outputs(args.dump_outputs, {"scores": (chain.fs, 0), "boxes": (chain.fb, 0), "classes": (chain.fc, 0)})
+            else:
+                last = pipes[(W + K - 1) % R]
+                dets = (last.fused.out, 7) if name == "v5s_b1" else (last.out, 17)
+                dump_outputs(args.dump_outputs, {"detections": dets, "net_input": (last.net_input, 0)})
         ms_e2e, win_e2e, nb2 = timed_blocks(step_e2e, K, W, stream, dev, 1, None)
         sampler.stop()
     fps, fps_e2e = B * K / (ms_dev * 1e-3), B * K / (ms_e2e * 1e-3)
@@ -1105,7 +1132,10 @@ def main():
     ap.add_argument("--force-gather", action="store_true", help="experiment: run the peer gather's publish + wait kernels at N = 1 too (this rank is its only peer)")
     ap.add_argument("--gather-no-wait", action="store_true", help="experiment: N > 1, publish only; the waits happen once at the end of a timed block (no flow control)")
     ap.add_argument("--fused-gather", action="store_true", help="N > 1: gather stores from inside nms_kernel + one-warp wait kernel")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "graft" or args.gpus > 1 or _env_int("WORLD_SIZE", 1) > 1 or args.force_gather):
+        ap.error("--dump-outputs: --impl graft on one GPU without the gather only")
     args.warmup = max(args.warmup, 3)
 
     rank, world, local_rank = _env_int("RANK", 0), _env_int("WORLD_SIZE", 1), _env_int("LOCAL_RANK", 0)

@@ -6,6 +6,7 @@ TEST INFRASTRUCTURE ONLY: imported by tests/, __graft_entry__.smoke() and bench.
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
 import subprocess
 from pathlib import Path
 
@@ -28,6 +29,19 @@ def load():
         subprocess.run(["make", "-C", str(HERE), str(LIB)], check=True, stdout=subprocess.DEVNULL)
     _lib = C.CDLL(str(LIB))
     return _lib
+
+
+def digest(a) -> str:
+    """sha256 of an array's dtype, shape and bytes: how golden files pin outputs that are compared bit for bit and are too
+    large to store (tests/golden/*.npz)."""
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).hexdigest()
+
+
+def sample_index(n: int, k: int = 64):
+    """The rows of an n-row output that golden files keep when the output is compared with a tolerance and is too large
+    to store whole: k of them (all when n <= k), ascending, fixed by n."""
+    return np.sort(np.random.default_rng(n).choice(n, min(n, k), replace=False))
 
 
 def _pp(arrs):

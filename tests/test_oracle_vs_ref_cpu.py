@@ -1,7 +1,8 @@
-"""Pins the oracle's NMS restatements against the REFERENCE's OWN host code: oracle/_ref/libref_*_host.so are
-built by oracle/Makefile from /root/reference/{yolov8,yolov5}/src/postprocess.cpp and retinaface/common.hpp,
-compiled where they lie (with header shims for the OpenCV / TensorRT includes those files pull in).
-The prebuilt libraries travel with the repo snapshot; these tests skip only if they were never built."""
+"""Pins the oracle's NMS restatements -- and the library's host functions -- against the REFERENCE's OWN host code
+({yolov8,yolov5}/src/postprocess.cpp and retinaface/common.hpp, compiled by oracle/Makefile with header shims for the
+OpenCV / TensorRT includes those files pull in).  What that code returned on the inputs below is stored in
+tests/golden/oracle_vs_ref.npz (tools/make_golden_vs_ref.py host): outputs as oracle.digest() strings, so every
+comparison stays bit for bit, on any machine."""
 import ctypes as C
 from pathlib import Path
 
@@ -10,34 +11,28 @@ import pytest
 
 from tensorrtx_b200 import synth
 
-REF = Path(__file__).resolve().parents[1] / "oracle" / "_ref"
+GOLD = Path(__file__).resolve().parent / "golden" / "oracle_vs_ref.npz"
 
 
-def _load(name):
-    p = REF / name
-    if not p.exists():
-        pytest.skip(f"{p} not built (run `make -C oracle` where /root/reference is mounted)")
-    return C.CDLL(str(p))
+@pytest.fixture(scope="module")
+def gold():
+    return np.load(GOLD)
 
 
-def _ref_nms(fn, buf, F, *thr):
-    out = np.zeros((buf.shape[0] // F + 1) * F, np.float32)
-    b = np.ascontiguousarray(buf, np.float32)
-    n = fn(b.ctypes.data_as(C.c_void_p), *[C.c_float(t) for t in thr], out.ctypes.data_as(C.c_void_p))
-    return out[:n * F].reshape(n, F).copy()
+def _same(oracle, gold, key, mine):
+    """`mine` is bit for bit what the reference's code returned (same rows, same order, same bits)."""
+    return oracle.digest(mine) == str(gold[key])
 
 
 @pytest.mark.parametrize("seed", range(4))
-def test_v8_nms_equals_reference(oracle, seed):
-    lib = _load("libref_yolov8_host.so")
-    assert lib.ref_v8_det_floats() == 90
+def test_v8_nms_equals_reference(oracle, gold, seed):
     heads = synth.yolov8_heads(2, seed=100 + seed)
     out, _ = oracle.yolov8_decode(heads)
     for b in range(2):
         mine, _ = oracle.nms(0, out[b], 1000, 90, 0.5, 0.45)
-        ref = _ref_nms(lib.ref_v8_nms, out[b], 90, 0.5, 0.45)
-        assert len(ref) > 20
-        assert np.array_equal(mine, ref)  # same rows, same order (class asc, conf desc), bit for bit
+        key = f"v8_nms_{seed}_{b}"
+        assert gold[key + "_n"] > 20
+        assert _same(oracle, gold, key, mine)  # same rows, same order (class asc, conf desc), bit for bit
 
 
 def _obb_plugin_rows(oracle, seed, B=2):
@@ -47,20 +42,18 @@ def _obb_plugin_rows(oracle, seed, B=2):
 
 
 @pytest.mark.parametrize("seed", range(3))
-def test_v8_nms_obb_equals_reference(oracle, seed):
+def test_v8_nms_obb_equals_reference(oracle, gold, seed):
     """nms_obb + probiou (mixed float/double C++ promotions): identical rows in identical order."""
-    lib = _load("libref_yolov8_host.so")
     out = _obb_plugin_rows(oracle, 130 + seed)
     for b in range(out.shape[0]):
         for thr in (0.5, 0.2):
             mine, _ = oracle.nms(3, out[b], 1000, 90, 0.3, thr)
-            ref = _ref_nms(lib.ref_v8_nms_obb, out[b], 90, 0.3, thr)
-            assert len(ref) > 10 and len(ref) < int(out[b, 0])
-            assert np.array_equal(mine, ref)
+            key = f"v8_obb_{seed}_{b}_{thr}"
+            assert gold[key + "_n"] > 10 and gold[key + "_n"] < int(out[b, 0])
+            assert _same(oracle, gold, key, mine)
 
 
-def test_v8_nms_ties_broken_by_bbox0_like_reference(oracle):
-    lib = _load("libref_yolov8_host.so")
+def test_v8_nms_ties_broken_by_bbox0_like_reference(oracle, gold):
     rng = np.random.default_rng(1)
     n = 400
     buf = np.zeros(1 + 1000 * 90, np.float32)
@@ -72,48 +65,36 @@ def test_v8_nms_ties_broken_by_bbox0_like_reference(oracle):
     rows[:, 5] = rng.integers(0, 3, n)
     buf[0] = n
     mine, _ = oracle.nms(0, buf, 1000, 90, 0.5, 0.45)
-    ref = _ref_nms(lib.ref_v8_nms, buf, 90, 0.5, 0.45)
-    assert np.array_equal(mine, ref)
+    assert _same(oracle, gold, "v8_ties", mine)
 
 
-def test_v8_batch_nms_and_thresholds(oracle):
-    lib = _load("libref_yolov8_host.so")
+def test_v8_batch_nms_and_thresholds(oracle, gold):
     heads = synth.yolov8_heads(3, seed=7)
     out, _ = oracle.yolov8_decode(heads)
-    res = np.zeros((3, 1000, 90), np.float32)
-    cnt = np.zeros(3, np.int32)
-    lib.ref_v8_batch_nms(np.ascontiguousarray(out).ctypes.data_as(C.c_void_p), 3, out.shape[1], C.c_float(0.3),
-                         C.c_float(0.6), res.ctypes.data_as(C.c_void_p), cnt.ctypes.data_as(C.c_void_p), 1000)
     for b in range(3):
         mine, _ = oracle.nms(0, out[b], 1000, 90, 0.3, 0.6)
-        assert cnt[b] == len(mine) and np.array_equal(res[b, :cnt[b]], mine)
+        assert gold[f"v8_batch_{b}_n"] == len(mine) and _same(oracle, gold, f"v8_batch_{b}", mine)
 
 
 @pytest.mark.parametrize("seed", range(3))
-def test_v5_nms_equals_reference(oracle, seed):
-    lib = _load("libref_yolov5_host.so")
-    assert lib.ref_v5_det_floats() == 38
+def test_v5_nms_equals_reference(oracle, gold, seed):
     heads = synth.yolov5_heads(1, seed=200 + seed, n_obj=200)
     out, _ = oracle.yolov5_decode(heads, synth.V5_ANCHORS)
     mine, _ = oracle.nms(1, out[0], 1000, 38, 0.5, 0.45)
-    ref = _ref_nms(lib.ref_v5_nms, out[0], 38, 0.5, 0.45)
-    assert len(ref) > 50 and np.array_equal(mine, ref)
+    assert gold[f"v5_nms_{seed}_n"] > 50 and _same(oracle, gold, f"v5_nms_{seed}", mine)
 
 
 @pytest.mark.parametrize("seed", range(3))
-def test_retina_nms_equals_reference(oracle, seed):
-    lib = _load("libref_retina_host.so")
+def test_retina_nms_equals_reference(oracle, gold, seed):
     heads = synth.retina_heads(1, seed=300 + seed, in_h=480, in_w=640, n_obj=60)
     out, _ = oracle.retina_decode(heads, in_h=480, in_w=640)
     tp = oracle.retina_total_priors(480, 640)
     mine, _ = oracle.nms(2, out[0], tp, 15, 0.1, 0.4)
-    ref = _ref_nms(lib.ref_retina_nms, out[0], 15, 0.4)
-    assert len(ref) > 20 and np.array_equal(mine, ref)
+    assert gold[f"retina_nms_{seed}_n"] > 20 and _same(oracle, gold, f"retina_nms_{seed}", mine)
 
 
-def test_retina_conf_threshold_is_a_double_compare(oracle):
+def test_retina_conf_threshold_is_a_double_compare(oracle, gold):
     """`output[..] <= 0.1` compares against the DOUBLE 0.1: conf == 0.1f (> 0.1) is kept (common.hpp:113)."""
-    lib = _load("libref_retina_host.so")
     tp = oracle.retina_total_priors(480, 640)
     buf = np.zeros(1 + tp * 15, np.float32)
     buf[0] = 3
@@ -121,66 +102,61 @@ def test_retina_conf_threshold_is_a_double_compare(oracle):
         buf[1 + i * 15:1 + i * 15 + 4] = [100 * i, 0, 100 * i + 50, 50]
         buf[1 + i * 15 + 4] = c
     mine, _ = oracle.nms(2, buf, tp, 15, 0.1, 0.4)
-    ref = _ref_nms(lib.ref_retina_nms, buf, 15, 0.4)
-    assert len(ref) == 2 and np.array_equal(mine, ref)
+    assert gold["retina_conf_n"] == 2 and _same(oracle, gold, "retina_conf", mine)
 
 
 @pytest.mark.parametrize("variant,libname,fn", [(0, "libref_yolov8_host.so", "ref_v8_get_rect"),
                                                 (1, "libref_yolov5_host.so", "ref_v5_get_rect")])
-def test_get_rect_equals_reference(oracle, variant, libname, fn):
+def test_get_rect_equals_reference(oracle, gold, variant, libname, fn):
     """get_rect (box in 640x640 network pixels -> cv::Rect in the original image): the reference's compiled host code vs
     the oracle vs the library's host function trtx_get_rect -- identical integers on 4000 boxes and 8 image sizes."""
     from tensorrtx_b200 import plugins as P
-    lib = _load(libname)
     rng = np.random.default_rng(50 + variant)
-    for (w, h) in ((1920, 1080), (1080, 1920), (640, 640), (1280, 720), (333, 777), (4000, 3000), (641, 640), (50, 60)):
+    rects = []
+    for (w, h) in SIZES:
         for _ in range(500):
             if variant == 0:
                 x1, y1 = rng.uniform(-30, 650, 2)
                 bb = np.array([x1, y1, x1 + rng.uniform(-5, 400), y1 + rng.uniform(-5, 400)], np.float32)
             else:
                 bb = np.array([rng.uniform(-30, 670), rng.uniform(-30, 670), rng.uniform(0, 500), rng.uniform(0, 500)], np.float32)
-            ref = np.zeros(4, np.int32)
-            getattr(lib, fn)(w, h, bb.ctypes.data_as(C.c_void_p), ref.ctypes.data_as(C.c_void_p))
-            assert np.array_equal(oracle.get_rect(variant, w, h, bb), ref)
-            assert P.get_rect(w, h, bb, variant=variant) == tuple(int(v) for v in ref)
-
+            r = oracle.get_rect(variant, w, h, bb)
+            assert P.get_rect(w, h, bb, variant=variant) == tuple(int(v) for v in r)
+            rects.append(r)
+    assert _same(oracle, gold, fn, np.array(rects))   # fn of the reference's library libname
 
 
 SIZES = ((1920, 1080), (1080, 1920), (640, 640), (1280, 720), (333, 777), (4000, 3000), (641, 640), (50, 60))
 
 
-def test_get_rect_adapt_landmark_equals_reference():
+def test_get_rect_adapt_landmark_equals_reference(oracle, gold):
     """get_rect_adapt_landmark (yolov8/src/postprocess.cpp:38-69, pose models): box AND the 17 keypoints mapped back to the
     original image -- the library's host function against the reference's compiled code, identical integers and identical
     keypoint bits on 300 boxes x 8 image sizes."""
     from tensorrtx_b200 import plugins as P
-    lib = _load("libref_yolov8_host.so")
     rng = np.random.default_rng(70)
+    rects, lmks = [], []
     for (w, h) in SIZES:
         for _ in range(300):
             x1, y1 = rng.uniform(-30, 650, 2)
             bb = np.array([x1, y1, x1 + rng.uniform(-5, 400), y1 + rng.uniform(-5, 400)], np.float32)
             lmk = rng.uniform(-20, 660, 51).astype(np.float32)
             lmk[2::3] = rng.uniform(0, 1, 17).astype(np.float32)
-            ref_l, ref_r = lmk.copy(), np.zeros(4, np.int32)
-            lib.ref_v8_get_rect_adapt_landmark(w, h, bb.copy().ctypes.data_as(C.c_void_p), ref_l.ctypes.data_as(C.c_void_p),
-                                               ref_r.ctypes.data_as(C.c_void_p))
             rect, mapped = P.get_rect_adapt_landmark(w, h, bb, lmk)
-            assert rect == tuple(int(v) for v in ref_r)
-            assert np.array_equal(np.asarray(mapped, np.float32), ref_l)
+            rects.append(np.array(rect, np.int32)), lmks.append(np.asarray(mapped, np.float32))
+    assert _same(oracle, gold, "v8_lmk_rects", np.array(rects))
+    assert _same(oracle, gold, "v8_lmk", np.array(lmks))
 
 
-def test_scale_mask_rect_and_process_decode_rows_equal_reference():
+def test_scale_mask_rect_and_process_decode_rows_equal_reference(gold):
     """scale_mask's crop of the 640x640 mask and its target size (postprocess.cpp:207-226; read back from the OpenCV shim) and
     process_decode_ptr_host (:131-147) -- the library's host functions against the reference's compiled code."""
     from tensorrtx_b200 import _lib as L
-    ref = _load("libref_yolov8_host.so")
     lib = L.load()
+    ref6 = iter(gold["scale_mask_rect"])
     for w in list(range(37, 2000, 97)) + [640, 641, 1920, 1080]:
         for h in (48, 479, 480, 640, 1080, 1920, 3000):
-            r6, mine = np.zeros(6, np.int32), (C.c_int * 4)()
-            ref.ref_v8_scale_mask_rect(w, h, r6.ctypes.data_as(C.c_void_p))
+            r6, mine = next(ref6), (C.c_int * 4)()
             assert lib.trtx_scale_mask_rect(640, 640, w, h, mine) == 0
             assert list(mine) == r6[:4].tolist() and r6[4:].tolist() == [w, h]
     rng = np.random.default_rng(71)
@@ -190,19 +166,15 @@ def test_scale_mask_rect_and_process_decode_rows_equal_reference():
     rows = buf[1:].reshape(K, 7)
     rows[:, :6] = rng.uniform(0, 640, (K, 6)).astype(np.float32)
     rows[:, 6] = rng.integers(0, 2, K)
-    out_ref, out_mine = np.zeros((K, 6), np.float32), np.zeros((K, 6), np.float32)
-    n_ref = ref.ref_v8_process_decode_ptr_host(buf.ctypes.data_as(C.c_void_p), 7, K, out_ref.ctypes.data_as(C.c_void_p))
+    out_ref, out_mine = gold["pdh"], np.zeros((K, 6), np.float32)
     n = lib.trtx_process_decode_ptr_host(buf.ctypes.data_as(C.POINTER(C.c_float)), 7, K, out_mine.ctypes.data_as(C.POINTER(C.c_float)))
-    assert n == n_ref == int(rows[:, 6].sum()) and np.array_equal(out_mine, out_ref)
+    assert n == len(out_ref) == int(rows[:, 6].sum()) and np.array_equal(out_mine[:n], out_ref)
 
 
-def test_process_decode_ptr_host_obb_equals_reference():
+def test_process_decode_ptr_host_obb_equals_reference(gold):
     """process_decode_ptr_host_obb (yolov8/src/postprocess.cpp:273-290): kept rows of the oriented-box compact buffer (8-float rows,
     angle in column 7) -- the library's host function against the reference's compiled code."""
     from tensorrtx_b200 import _lib as L
-    ref = _load("libref_yolov8_host.so")
-    if not hasattr(ref, "ref_v8_process_decode_ptr_host_obb"):
-        pytest.skip("oracle/_ref predates the obb wrapper (run `make -C oracle` where /root/reference is mounted)")
     lib = L.load()
     rng = np.random.default_rng(72)
     for elem in (8, 9):
@@ -212,33 +184,29 @@ def test_process_decode_ptr_host_obb_equals_reference():
         rows = buf[1:].reshape(K, elem)
         rows[:, :] = rng.uniform(-3, 640, (K, elem)).astype(np.float32)
         rows[:, 6] = rng.integers(0, 3, K)                  # keep flags 0, 1, 2: only == 1 is kept
-        out_ref, out_mine = np.zeros((K, 7), np.float32), np.zeros((K, 7), np.float32)
-        n_ref = ref.ref_v8_process_decode_ptr_host_obb(buf.ctypes.data_as(C.c_void_p), elem, K, out_ref.ctypes.data_as(C.c_void_p))
+        out_ref, out_mine = gold[f"pdh_obb_{elem}"], np.zeros((K, 7), np.float32)
         n = lib.trtx_process_decode_ptr_host_obb(buf.ctypes.data_as(C.POINTER(C.c_float)), elem, K, out_mine.ctypes.data_as(C.POINTER(C.c_float)))
-        assert n == n_ref == int((rows[:, 6] == 1).sum()) and n > 20 and np.array_equal(out_mine, out_ref)
+        assert n == len(out_ref) == int((rows[:, 6] == 1).sum()) and n > 20 and np.array_equal(out_mine[:n], out_ref)
     assert lib.trtx_process_decode_ptr_host_obb(buf.ctypes.data_as(C.POINTER(C.c_float)), 7, K, out_mine.ctypes.data_as(C.POINTER(C.c_float))) < 0
 
 
-def test_retina_get_rect_adapt_landmark_equals_reference():
+def test_retina_get_rect_adapt_landmark_equals_reference(oracle, gold):
     """RetinaFace's get_rect_adapt_landmark (retinaface/common.hpp:65-89: box corners truncated to int, 5 landmark pairs mapped in
     place) -- the library's host function against the reference's compiled code: identical integers and landmark bits on 250 faces
     x 8 image sizes, for the 640x640 network of BASELINE config 3 and the 480x640 one the reference compiles in."""
     from tensorrtx_b200 import _lib as L
-    ref = _load("libref_retina_host.so")
-    if not hasattr(ref, "ref_retina_get_rect_adapt_landmark"):
-        pytest.skip("oracle/_ref predates this wrapper (run `make -C oracle` where /root/reference is mounted)")
     lib = L.load()
     rng = np.random.default_rng(73)
+    rects, lmks = [], []
     for (in_w, in_h) in ((640, 640), (640, 480)):
         for (w, h) in SIZES:
             for _ in range(250):
                 x1, y1 = rng.uniform(-30, in_w + 10), rng.uniform(-30, in_h + 10)
                 bb = np.array([x1, y1, x1 + rng.uniform(-5, 400), y1 + rng.uniform(-5, 400)], np.float32)
                 lmk = rng.uniform(-20, 660, 10).astype(np.float32)
-                l_ref, r_ref = lmk.copy(), np.zeros(4, np.int32)
-                ref.ref_retina_get_rect_adapt_landmark(w, h, in_w, in_h, bb.copy().ctypes.data_as(C.c_void_p), l_ref.ctypes.data_as(C.c_void_p),
-                                                       r_ref.ctypes.data_as(C.c_void_p))
                 l_mine, r_mine = lmk.copy(), (C.c_int * 4)()
                 assert lib.trtx_retina_get_rect_adapt_landmark(in_w, in_h, w, h, bb.ctypes.data_as(C.POINTER(C.c_float)),
                                                                l_mine.ctypes.data_as(C.POINTER(C.c_float)), r_mine) == 0
-                assert list(r_mine) == r_ref.tolist() and np.array_equal(l_mine, l_ref)
+                rects.append(np.array(list(r_mine), np.int32)), lmks.append(l_mine)
+    assert _same(oracle, gold, "retina_lmk_rects", np.array(rects))
+    assert _same(oracle, gold, "retina_lmk", np.array(lmks))
