@@ -107,6 +107,9 @@ typedef struct trtx_yolo_params {
     int32_t tune_tma_pipeline;   /* 1: persistent TMA-fed scan (v8 layout, 16-byte aligned levels); 0 = register scan */
     int32_t tune_tma_stages;     /* cap on its pipeline stages; 0 = as many as fit (15) */
     int32_t tune_box_prefetch;   /* box rows of a tile: 1 on demand, 2 L2 prefetch, 3 into registers up front; 0 = 2 */
+    int32_t tune_nms_threads;    /* threads per NMS CTA of the fused / split decode + NMS calls: 1024 (every case) or 512
+                                    (half an SM: greedy mode, axis-aligned boxes, max_out <= 1024, no gather fused into
+                                    the NMS); 0 = 1024.  Both give identical outputs. */
 } trtx_yolo_params;
 
 /* Fill grid_h/grid_w from net size and strides (v8) -- convenience, mirrors yololayer.cu:292-296. */

@@ -52,6 +52,7 @@ class YoloParams(C.Structure):
         ("tune_tma_pipeline", C.c_int32),
         ("tune_tma_stages", C.c_int32),
         ("tune_box_prefetch", C.c_int32),
+        ("tune_nms_threads", C.c_int32),
     ]
 
 

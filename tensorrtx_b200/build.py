@@ -47,7 +47,8 @@ def _stamp(sources: list[Path]) -> str:
 def build(force: bool = False, verbose: bool = False, probe: bool = False, defines: tuple = (), suffix: str = "") -> Path:
     """Compile every CUDA source for sm_100a into tensorrtx_b200/lib/libtrtx_hot.so.
     probe=True builds libtrtx_hot_probe.so instead: the same sources with -DTRTX_NMS_PROBE (clock64 phase stamps in
-    nms_kernel + trtx_probe_set_nms_stamps), used by tools/nms_probe.py only.  `defines` + `suffix`: further experiment
+    nms_kernel + trtx_probe_set_nms_stamps, used by tools/nms_probe.py; per-CTA %globaltimer stamps of the scan, NMS and
+    letterbox kernels + trtx_probe_set_timeline, used by tools/step_timeline.py).  `defines` + `suffix`: further experiment
     builds (tools/scan_probe.py), never loaded by the product path."""
     srcs = [CSRC / s for s in SOURCES if (CSRC / s).exists()]
     LIBDIR.mkdir(exist_ok=True)

@@ -13,6 +13,49 @@ constexpr size_t kAlign = 256;  // workspace sub-buffer alignment (rcnn/cuda_uti
 
 __host__ __device__ inline size_t align_up(size_t v, size_t a = kAlign) { return (v + a - 1) / a * a; }
 
+// ---- step timeline (probe build only: build(probe=True) / -DTRTX_NMS_PROBE; release builds carry no stamps) ----
+// Every launch of the scan, NMS and letterbox kernels takes the next record of the buffer registered with
+// trtx_probe_set_timeline (this host thread's launches, in launch order; null once the buffer is full) through its
+// argument block.  Record: [kind, CTAs, then per CTA (first %globaltimer stamp at entry, last stamp at exit)], in ns.
+// The caller zeroes the buffer before each run (exit stamps are atomic maxima).
+#ifdef TRTX_NMS_PROBE
+enum TlKind { kTlScan = 1, kTlNms = 2, kTlLetterbox = 3 };
+constexpr int kTlMaxCtas = 8192;
+constexpr size_t kTlRecordWords = 2 + 2 * (size_t)kTlMaxCtas;
+unsigned long long* tl_take();  // nms.cu
+__device__ __forceinline__ unsigned long long tl_now() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+struct TlStamp {
+    unsigned long long* r;
+    __device__ __forceinline__ TlStamp(unsigned long long* rec, int kind) : r(nullptr) {
+        const unsigned ncta = gridDim.x * gridDim.y * gridDim.z;
+        if (!rec || ncta > (unsigned)kTlMaxCtas) return;
+        const unsigned cta = blockIdx.x + gridDim.x * (blockIdx.y + gridDim.y * blockIdx.z);
+        r = rec + 2 + 2 * (size_t)cta;
+        if (threadIdx.x + threadIdx.y + threadIdx.z == 0) {
+            r[0] = tl_now();
+            if (cta == 0) {
+                rec[0] = (unsigned long long)kind;
+                rec[1] = ncta;
+            }
+        }
+    }
+    __device__ __forceinline__ ~TlStamp() {  // runs at every return: one atomic max per (warp, exit point)
+        if (r && (threadIdx.x & 31) == (unsigned)(__ffs(__activemask()) - 1)) atomicMax(r + 1, tl_now());
+    }
+};
+#define TRTX_TL_FIELD unsigned long long* tl;
+#define TRTX_TL(args, kind) TlStamp tl_stamp_((args).tl, (kind))
+#define TRTX_TL_TAKE(args) ((args).tl = tl_take())
+#else
+#define TRTX_TL_FIELD
+#define TRTX_TL(args, kind) do { } while (0)
+#define TRTX_TL_TAKE(args) do { } while (0)
+#endif
+
 // thread-local last CUDA error (trtx_last_cuda_error)
 extern thread_local int g_last_cuda_error;
 inline int check_launch() {

@@ -1,5 +1,5 @@
-// nms.cu -- sort + class-aware greedy NMS, one 1024-thread CTA per image, every image of the batch
-// in one launch.  Replaces
+// nms.cu -- sort + class-aware greedy NMS, one CTA (1024 threads; 512 on request on the fused YOLO path) per
+// image, every image of the batch in one launch.  Replaces
 //   host  nms()/batch_nms()      yolov8/src/postprocess.cpp:94-129, yolov5/src/postprocess.cpp:49-80,
 //                                retinaface/common.hpp:110-130           (std::map + std::sort + erase)
 //   device cuda_decode()+cuda_nms()  yolov8/src/postprocess.cu:42-111,168-179   (batch 1 only, one-shot)
@@ -9,16 +9,16 @@
 //   B  if more than `pre_topk` survive: block radix-select (4 x 8-bit passes) of the top pre_topk,
 //      ties at the cut broken by the smaller id (second radix select over the ids)
 //   C  bitonic sort by (class asc, conf desc, box[0] asc, id asc) -- the order the reference builds with
-//      std::map<float,...> + std::sort(cmp).  Up to 1024 rows: one row per thread in registers, the
-//      j < 32 exchange steps are warp shuffles, only the 15 j >= 32 steps go through shared memory
-//      (1 barrier each, ping-pong buffers); up to 2048 rows: plain shared-memory network.
+//      std::map<float,...> + std::sort(cmp).  Up to one row per thread: rows in registers, the
+//      j < 32 exchange steps are warp shuffles, only the j >= 32 steps go through shared memory
+//      (1 barrier each, ping-pong buffers); more rows: plain shared-memory network.
 //   D  stage boxes of the sorted rows in shared memory (SoA)
 //   E  greedy NMS per CLASS SEGMENT of the sorted list (rows of different classes never interact):
 //      short segments (<= 96 rows, the normal multi-class case) are claimed by single warps and
 //      resolved with shuffles + ballots only -- no block barrier at all;  long segments (single-class
 //      models such as retinaface, or degenerate inputs) are processed by the whole CTA in chunks of 32
-//      rows: every chunk member is tested against the already-kept rows (all 1024 threads, IoU tile in
-//      shared memory) and against its 31 chunk-mates (warp w = member w, lane j = mate j, one
+//      rows: every chunk member is tested against the already-kept rows (all threads, IoU tile in
+//      shared memory) and against its 31 chunk-mates (warp w = member w mod warps, lane j = mate j, one
 //      __ballot_sync per member gives its suppressor bitmap); warp 0 resolves the chunk serially on
 //      the 32x32 bitmap.  2 barriers per 32 rows.
 //   F  block scan of the keep flags -> [count, (box, conf, cls, keep, extras)*] in sorted order.
@@ -35,14 +35,28 @@ namespace trtx {
 // tools/nms_probe.py): the release library has no profiling state at all.
 #ifdef TRTX_NMS_PROBE
 static thread_local long long* t_nms_stamps = nullptr;
+static thread_local unsigned long long* t_tl_buf = nullptr;
+static thread_local int t_tl_records = 0, t_tl_next = 0;
+unsigned long long* tl_take() {
+    if (!t_tl_buf || t_tl_next >= t_tl_records) return nullptr;
+    return t_tl_buf + kTlRecordWords * (size_t)t_tl_next++;
+}
 #define TRTX_STAMP(k) do { if (a.dbg && threadIdx.x == 0) a.dbg[blockIdx.x * 16 + (k)] = clock64(); } while (0)
 #else
 #define TRTX_STAMP(k) do { } while (0)
 #endif
 
+// Block sizes of nms_kernel.  The general kernel (every source, box format and mode, up to kMaxSort rows) runs 1024
+// threads at 60 registers, so it needs an SM of its own.  The half-SM instantiation (512 threads, <= 64 registers, 2 CTAs
+// an SM by launch bounds) fits next to 5 letterbox or 8 scan CTAs; it covers the fused YOLO path (tile source, greedy,
+// axis-aligned, pre_topk <= 1024, no fused gather) on request (trtx_yolo_params.tune_nms_threads = 512).  Both compute
+// the same outputs: only the mapping of threads to work differs.  It is not the default: on a B200 at b32 its CTAs run
+// 30-35 us next to the streaming letterbox instead of 21-24 (half the threads for the same phases), which costs more
+// than placing a CTA early gains (profiles/r03a_timeline_*.log).
 constexpr int kNmsThreads = 1024;
+constexpr int kNmsThreadsHalf = 512;
 constexpr int kMaxSort = TRTX_NMS_MAX_ROWS;  // rows entering NMS per image (>= kMaxNumOutputBbox = 1000)
-constexpr int kClassBins = kNmsThreads;  // bucket sort: one histogram bin per thread
+// bucket sort: one histogram bin per thread (NT bins; a class id >= NT takes the bitonic paths)
 constexpr int kMaxBucket = 256;           // rows per class the rank-by-counting pass accepts
 constexpr int kShortSeg = 96;  // class segments up to this many rows are resolved by a single warp
 
@@ -71,6 +85,7 @@ struct NmsArgs {
 #ifdef TRTX_NMS_PROBE
     long long* dbg;       // 16 clock64 stamps per image, or null
 #endif
+    TRTX_TL_FIELD  // probe build: this launch's timeline record
     float* out;           // [B, 1 + max_det*(7+extra)]
     int32_t* keep_index;  // [B, max_det] or null
     // multi-GPU: phase F also stores every emitted row (and the count) into the gathered buffer of EVERY rank over
@@ -254,7 +269,15 @@ __device__ __forceinline__ int seg_units(int m) {
     return G * (m - 1) - 4 * G * (G - 1);
 }
 
-__global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_constant__ NmsArgs a) {
+template <int NT>
+__global__ void __launch_bounds__(NT, kNmsThreads / NT) nms_kernel(const __grid_constant__ NmsArgs a) {
+    constexpr int NW = NT / 32;  // warps; per-warp partials in s_wsum[0 .. NW)
+    static_assert(NT % 32 == 0 && NT >= 256 && NT <= 1024, "the 256-bin histograms need >= 256 threads");
+    // Programmatic dependent launch (nms_launch): this CTA may become resident while the kernel before it in the stream
+    // still runs.  Nothing before this point touches global memory; the wait returns once that kernel has completed
+    // and its writes are visible (a no-op after an ordinary launch).
+    TRTX_TL(a, kTlNms);  // entry stamp = the CTA is resident (under PDL: possibly before the scan has completed)
+    asm volatile("griddepcontrol.wait;" ::: "memory");
     extern __shared__ __align__(16) unsigned char smem_raw[];
     // carve-up (S = row capacity, power of two >= pre_topk)
     const int S = a.pre_topk <= 1024 ? 1024 : kMaxSort;
@@ -282,7 +305,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
     unsigned long long* k_lo = k_hi + S;
 
     __shared__ int s_hist[256];
-    __shared__ int s_chist[kClassBins], s_cstart[kClassBins];  // bucket sort: rows per class, first sorted row of a class
+    __shared__ int s_chist[NT], s_cstart[NT];  // bucket sort: rows per class, first sorted row of a class
     __shared__ int s_n, s_need, s_bucket, s_nkept, s_nshort, s_nmed, s_nlong, s_cursor, s_bad, s_nunit;
     __shared__ unsigned s_rem;
     __shared__ unsigned s_sup[32];
@@ -317,7 +340,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
         const int T = a.tiles_per_image;
         const int* cnt = a.tile_count + (size_t)b * T;
         int carry = 0;
-        for (int base = 0; base < T; base += kNmsThreads) {
+        for (int base = 0; base < T; base += NT) {
             const int t = base + tid;
             const int v = t < T ? cnt[t] : 0;
             int tot;
@@ -325,7 +348,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
             if (lane == 0) s_wsum[warp] = tot;
             __syncthreads();
             if (warp == 0) {
-                int w = s_wsum[lane], wt;
+                int w = lane < NW ? s_wsum[lane] : 0, wt;
                 const int wex = warp_excl_scan(w, lane, &wt);
                 s_wsum[lane] = wex;
                 if (lane == 0) s_need = wt;
@@ -341,7 +364,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
         // nms() filters THOSE by confidence: same here with "first" = ascending anchor order (what
         // trtx_yolo_decode_enqueue + trtx_nms_enqueue do through the plugin buffer), so both paths agree above max_out.
         const int n_in = min(carry, a.pre_topk);
-        for (int r = tid; r < n_in; r += kNmsThreads) {
+        for (int r = tid; r < n_in; r += NT) {
             int lo = 0, hi = T;  // largest t with s_tpre[t] <= r
             while (hi - lo > 1) {
                 const int mid = (lo + hi) >> 1;
@@ -359,7 +382,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
         const float* img = a.rows + (size_t)b * (1 + (size_t)a.max_rows * a.det_floats);
         int n_in = (int)img[0];  // `i < output[0]`
         n_in = max(0, min(n_in, a.max_rows));
-        for (int i = tid; i < n_in; i += kNmsThreads) {
+        for (int i = tid; i < n_in; i += NT) {
             const Row row = fetch_row(a, b, (uint32_t)i);
             if (a.mode == TRTX_NMS_ONESHOT ? row.conf >= a.conf_thresh : row.conf > a.conf_thresh) stash(row, (uint32_t)i);
         }
@@ -377,7 +400,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
             const int shift = 24 - 8 * pass;
             if (tid < 256) s_hist[tid] = 0;
             __syncthreads();
-            for (int i = tid; i < n_valid; i += kNmsThreads) {
+            for (int i = tid; i < n_valid; i += NT) {
                 uint32_t k = list[i].x;
                 if ((k & mask) == prefix) atomicAdd(&s_hist[(k >> shift) & 255], 1);
             }
@@ -401,7 +424,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
             const int shift = 24 - 8 * pass;
             if (tid < 256) s_hist[tid] = 0;
             __syncthreads();
-            for (int i = tid; i < n_valid; i += kNmsThreads) {
+            for (int i = tid; i < n_valid; i += NT) {
                 uint2 e = list[i];
                 if (e.x == key_cut && (e.y & im) == ip) atomicAdd(&s_hist[(e.y >> shift) & 255], 1);
             }
@@ -423,7 +446,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
             s_bad = 0;
         }
         __syncthreads();
-        for (int i = tid; i < n_valid; i += kNmsThreads) {
+        for (int i = tid; i < n_valid; i += NT) {
             const uint2 e = list[i];
             if (e.x > key_cut || (e.x == key_cut && e.y <= id_cut)) {
                 const Row r = fetch_row(a, b, e.y);
@@ -448,22 +471,22 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
     bool generic = s_bad != 0;
     // fastest path (the detector case: many classes, a few dozen rows each): counting sort by class, then every row
     // ranks itself inside its class bucket by counting smaller keys -- no compare-exchange network.
-    // Falls through to the bitonic paths when a class id is >= kClassBins or a bucket holds more than kMaxBucket rows.
+    // Falls through to the bitonic paths when a class id is >= NT or a bucket holds more than kMaxBucket rows.
     bool bucketed = false;
     if (!generic) {
         unsigned long long* kb = reinterpret_cast<unsigned long long*>(s_box);  // keys in bucket order (rows not staged yet)
         s_chist[tid] = 0;
         __syncthreads();
         bool big = false;
-        for (int base = 0; base < M; base += kNmsThreads) {
+        for (int base = 0; base < M; base += NT) {
             // rows arrive in tile order, so neighbouring lanes often share a class: one atomic per (warp, class)
             const int i = base + tid;
             const int c = i < M ? u_cls[i] : -1;
             const unsigned peers = __match_any_sync(0xffffffffu, c);
             const int leader = __ffs(peers) - 1;
             int first = 0;
-            if (c >= kClassBins) big = true;
-            if (lane == leader && c >= 0 && c < kClassBins) first = atomicAdd(&s_chist[c], __popc(peers));
+            if (c >= NT) big = true;
+            if (lane == leader && c >= 0 && c < NT) first = atomicAdd(&s_chist[c], __popc(peers));
             first = __shfl_sync(0xffffffffu, first, leader);
             if (i < M) s_pos[i] = (unsigned short)(first + __popc(peers & ((1u << lane) - 1u)));  // slot inside the bucket (any order works)
         }
@@ -474,21 +497,21 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
         if (lane == 0) s_wsum[warp] = tot;
         if (!__syncthreads_or(big || h > kMaxBucket ? 1 : 0)) {
             if (warp == 0) {
-                int w = s_wsum[lane], wt;
+                int w = lane < NW ? s_wsum[lane] : 0, wt;
                 const int wex = warp_excl_scan(w, lane, &wt);
                 s_wsum[lane] = wex;
             }
             __syncthreads();
             s_cstart[tid] = s_wsum[warp] + ex;
             __syncthreads();
-            for (int i = tid; i < M; i += kNmsThreads) {
+            for (int i = tid; i < M; i += NT) {
                 const int c = u_cls[i];
                 kb[s_cstart[c] + s_pos[i]] =
                     ((unsigned long long)(uint32_t)c << 48) | ((unsigned long long)(uint32_t)(~float_key(u_conf[i])) << 16) | (uint32_t)i;
             }
             __syncthreads();
             // thread p owns bucket slot p: neighbouring lanes share a bucket, so the key reads below are broadcasts
-            for (int p = tid; p < M; p += kNmsThreads) {
+            for (int p = tid; p < M; p += NT) {
                 const unsigned long long mk = kb[p];
                 const int c = (int)(mk >> 48);
                 const int s0 = s_cstart[c], m = s_chist[c];
@@ -499,18 +522,18 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
             }
             __syncthreads();
             bool tie = false;  // same (class, conf) twice: the generic sort decides by (box[0], id)
-            for (int i = tid; i < M; i += kNmsThreads)
+            for (int i = tid; i < M; i += NT)
                 if (i > 0 && (k64[i] >> 16) == (k64[i - 1] >> 16)) tie = true;
             generic = __syncthreads_or(tie ? 1 : 0) != 0;
             bucketed = !generic;
         }
     }
     if (!generic && !bucketed) {
-        for (int i = tid; i < S_eff; i += kNmsThreads)
+        for (int i = tid; i < S_eff; i += NT)
             k64[i] = i < M ? ((unsigned long long)(uint32_t)u_cls[i] << 48) | ((unsigned long long)(uint32_t)(~float_key(u_conf[i])) << 16) | (uint32_t)i
                            : ~0ull;
         __syncthreads();
-        if (S_eff <= kNmsThreads) {
+        if (S_eff <= NT) {
             // one key per thread in registers; shuffles for partner distance < 32, smem ping-pong otherwise
             unsigned long long* ex = reinterpret_cast<unsigned long long*>(s_box);  // 2 x 1024 u64 scratch (rows not staged yet)
             unsigned long long mk = tid < S_eff ? k64[tid] : ~0ull;
@@ -519,9 +542,9 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
                 for (int jj = k >> 1; jj > 0; jj >>= 1) {
                     unsigned long long ok;
                     if (jj >= 32) {
-                        ex[pp * kNmsThreads + tid] = mk;
+                        ex[pp * NT + tid] = mk;
                         __syncthreads();
-                        ok = ex[pp * kNmsThreads + (tid ^ jj)];
+                        ok = ex[pp * NT + (tid ^ jj)];
                         pp ^= 1;
                     } else {
                         ok = __shfl_xor_sync(0xffffffffu, mk, jj);
@@ -536,7 +559,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
         } else {
             for (int k = 2; k <= S_eff; k <<= 1) {
                 for (int jj = k >> 1; jj > 0; jj >>= 1) {
-                    for (int i = tid; i < S_eff; i += kNmsThreads) {
+                    for (int i = tid; i < S_eff; i += NT) {
                         const int ixj = i ^ jj;
                         if (ixj > i) {
                             const unsigned long long x = k64[i], y = k64[ixj];
@@ -551,12 +574,12 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
             }
         }
         bool tie = false;
-        for (int i = tid; i < M; i += kNmsThreads)
+        for (int i = tid; i < M; i += NT)
             if (i > 0 && (k64[i] >> 16) == (k64[i - 1] >> 16)) tie = true;
         generic = __syncthreads_or(tie ? 1 : 0) != 0;
     }
     if (generic) {
-        for (int i = tid; i < S_eff; i += kNmsThreads) {
+        for (int i = tid; i < S_eff; i += NT) {
             if (i < M) {
                 k_hi[i] = ((unsigned long long)(uint32_t)u_cls[i] << 32) | (uint32_t)(~float_key(u_conf[i]));
                 k_lo[i] = ((unsigned long long)(a.tie_break_x0 ? float_key(u_box[i].x) : 0u) << 32) | u_id[i];
@@ -569,7 +592,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
         __syncthreads();
         for (int k = 2; k <= S_eff; k <<= 1) {
             for (int jj = k >> 1; jj > 0; jj >>= 1) {
-                for (int i = tid; i < S_eff; i += kNmsThreads) {
+                for (int i = tid; i < S_eff; i += NT) {
                     const int ixj = i ^ jj;
                     if (ixj > i) {
                         const unsigned long long ah = k_hi[i], al = k_lo[i], bh = k_hi[ixj], bl = k_lo[ixj];
@@ -588,7 +611,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
                 __syncthreads();
             }
         }
-        for (int i = tid; i < M; i += kNmsThreads) k64[i] = s_pos[i];  // permutation in the low 16 bits, like the fast path
+        for (int i = tid; i < M; i += NT) k64[i] = s_pos[i];  // permutation in the low 16 bits, like the fast path
         __syncthreads();  // the 128-bit keys (in the sorted-row area) are dead from here on
     }
 
@@ -601,7 +624,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
     iq.retina = a.box_format == TRTX_BOX_RETINA;
     iq.zero_hit = 0.0f > a.nms_thresh;
     iq.fast_ok = fabsf(a.nms_thresh) <= 4.0f;
-    for (int i = tid; i < M; i += kNmsThreads) {
+    for (int i = tid; i < M; i += NT) {
         const int pos = (int)(k64[i] & 0xffffull);
         const float4 bx = u_box[pos];
         if (a.box_format == TRTX_BOX_OBB) {  // covariance of the row's Gaussian, once per row; the angle is the first extra float
@@ -648,7 +671,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
         // ---------------- E: class segments ----------------
         if (bucketed) {
             // the class histogram already is the segment table
-            for (int i = tid; i < M; i += kNmsThreads) {
+            for (int i = tid; i < M; i += NT) {
                 const int c = s_cls[i], m = s_chist[c];
                 s_rowseg[i] = m > kShortSeg ? 0 : ((s_cstart[c] << 16) | m);
             }
@@ -661,7 +684,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
                 s_seg[atomicAdd(&s_nshort, 1)] = (p0 << 16) | m;
             if (m > 1 && m <= kShortSeg) s_pos[p0] = (unsigned short)atomicAdd(&s_nunit, seg_units(m));
         } else
-        for (int i = tid; i < M; i += kNmsThreads) {
+        for (int i = tid; i < M; i += NT) {
             if (i == 0 || s_cls[i] != s_cls[i - 1]) {
                 int e = i + 1;
                 while (e < M && s_cls[e] == s_cls[i]) ++e;
@@ -687,14 +710,14 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
             for (int c0 = 0; c0 < m; c0 += 32) {
                 const int nchunk = min(32, m - c0);
                 const int P = 32 * n_kept;
-                for (int p = tid; p < P; p += kNmsThreads) {
+                for (int p = tid; p < P; p += NT) {
                     const int i = p & 31, k = p >> 5;
                     const int kr = s_krow[k];
                     if (i < nchunk && overlaps(iq, s_box[kr], s_area[kr], s_box[p0 + c0 + i], s_area[p0 + c0 + i]))
                         atomicOr(&s_rem, 1u << i);
                 }
-                {
-                    const int i = warp, jx = lane;
+                for (int i = warp; i < 32; i += NW) {  // chunk member i: warp i % NW, lane = mate
+                    const int jx = lane;
                     bool hit = false;
                     if (i < nchunk && jx < i)
                         hit = overlaps(iq, s_box[p0 + c0 + jx], s_area[p0 + c0 + jx], s_box[p0 + c0 + i], s_area[p0 + c0 + i]);
@@ -729,10 +752,10 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
         // ---- short / medium segments (<= kShortSeg rows) ----
         // (1) IoU of every row against the earlier rows of its segment -> suppressor bitmap per row (bit j = row start+j
         //     overlaps it).  Work unit = (row, group g of 8 earlier rows) = one byte of the bitmap.  The units of all
-        //     segments go into one list so the 1024 threads share them evenly whatever the segment lengths are; inside
+        //     segments go into one list so the threads share them evenly whatever the segment lengths are; inside
         //     a segment they are ordered group-major, so neighbouring lanes hold neighbouring rows and test them
         //     against the SAME 8 earlier rows (shared-memory broadcasts instead of 128-byte-stride bank conflicts).
-        for (int i = tid; i < M; i += kNmsThreads) {
+        for (int i = tid; i < M; i += NT) {
             const int rs = s_rowseg[i];
             if (rs == 0) continue;
             const int p0 = rs >> 16, m = rs & 0xffff, li = i - p0;
@@ -747,7 +770,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
         {
             const int n_unit = s_nunit;
             unsigned char* mask_bytes = reinterpret_cast<unsigned char*>(s_mask);
-            for (int u = tid; u < n_unit; u += kNmsThreads) {
+            for (int u = tid; u < n_unit; u += NT) {
                 const int e = s_unit[u], i = e >> 4, g = e & 15;
                 const int p0 = s_rowseg[i] >> 16, li = i - p0;
                 const float4 bi = s_box[i];
@@ -802,7 +825,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
         __syncthreads();
     } else {
         // one-shot: dropped iff some earlier same-class row (higher conf) overlaps (postprocess.cu:89-111)
-        for (int i = tid; i < M; i += kNmsThreads) {
+        for (int i = tid; i < M; i += NT) {
             const int ci = s_cls[i];
             const float4 bi = s_box[i];
             bool keep = true;
@@ -822,14 +845,14 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
     // ---------------- F: block scan of the output flags, rows in sorted (class, conf) order ----------------
     // greedy: only kept rows are emitted; one-shot: every row is emitted with its keep flag
     int carry = 0;
-    for (int base = 0; base < M; base += kNmsThreads) {
+    for (int base = 0; base < M; base += NT) {
         const int i = base + tid;
         const bool emit = i < M && (a.mode == TRTX_NMS_ONESHOT || s_keep[i]);
         const unsigned bal = __ballot_sync(0xffffffffu, emit);
         if (lane == 0) s_wsum[warp] = __popc(bal);
         __syncthreads();
         if (warp == 0) {
-            int v = s_wsum[lane], tot;
+            int v = lane < NW ? s_wsum[lane] : 0, tot;
             const int ex = warp_excl_scan(v, lane, &tot);
             s_wsum[lane] = ex;
             if (lane == 0) s_nkept = tot;
@@ -863,9 +886,9 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
     const int n_rows_out = min(carry, a.max_det);
     if (tid == 0) o[0] = (float)n_rows_out;
     // rows >= count are zero (the reference memsets its decode buffer, yolov8_det.cpp:106)
-    for (int i = n_rows_out * R + tid; i < a.max_det * R; i += kNmsThreads) o[1 + i] = 0.0f;
+    for (int i = n_rows_out * R + tid; i < a.max_det * R; i += NT) o[1 + i] = 0.0f;
     if (oidx)
-        for (int i = n_rows_out + tid; i < a.max_det; i += kNmsThreads) oidx[i] = -1;
+        for (int i = n_rows_out + tid; i < a.max_det; i += NT) oidx[i] = -1;
     if (gworld) {
         // The image's block [count, rows...] is contiguous and was just written to `o` by this CTA: copy its live part to every
         // rank's gathered buffer with lane-consecutive stores (full 128-byte NVLink writes instead of one 4-byte packet per
@@ -874,7 +897,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const __grid_consta
         const int live = 1 + n_rows_out * R;
         for (int p = 0; p < gworld; ++p) {
             float* dstp = a.g.out[p] + goff;
-            for (int i = tid; i < live; i += kNmsThreads) dstp[i] = i == 0 ? (float)n_rows_out : o[i];
+            for (int i = tid; i < live; i += NT) dstp[i] = i == 0 ? (float)n_rows_out : o[i];
         }
         __syncthreads();  // CTA-scope order of all peer stores before thread 0's system-scope fence (cumulative)
         if (tid == 0) {
@@ -980,18 +1003,61 @@ static int nms_validate(const trtx_nms_params* q) {
     return TRTX_OK;
 }
 
-static int nms_launch(NmsArgs& a, int batch, cudaStream_t st) {
+// The half-SM kernel covers the fused YOLO source in greedy mode with axis-aligned boxes and at most 1024 rows, without
+// the gather fused into the kernel.
+static bool nms_half_ok(const NmsArgs& a) {
+    return a.from_tiles && a.mode == TRTX_NMS_GREEDY && a.box_format != TRTX_BOX_OBB && a.pre_topk <= 1024 && a.g.world == 0;
+}
+
+template <int NT>
+static cudaError_t nms_launch_nt(const NmsArgs& a, int batch, size_t smem, cudaStream_t st) {
+    // per-device function attribute; cheap and idempotent, so set on every call (no global state).
+    // 227 KB per CTA minus the kernel's static shared memory (histograms, <= ~18 KB)
+    constexpr size_t kMaxDynSmem = (227 - 20) * 1024;
+    cudaFuncSetAttribute(nms_kernel<NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxDynSmem);
+    // Programmatic dependent launch: the CTAs may be placed (and run up to griddepcontrol.wait) while the previous kernel
+    // of the stream -- the scan, which triggers once its streaming loop is done -- finishes its tail, instead of after
+    // it.  Stream capture turns the attribute into a programmatic graph edge.
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3(batch);
+    cfg.blockDim = dim3(NT);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = at;
+    cfg.numAttrs = 1;
+#ifdef TRTX_NMS_NO_PDL  // experiment build (tools/step_timeline.py): the ordinary launch, for before / after timelines
+    cfg.numAttrs = 0;
+#endif
+    cudaError_t e = cudaLaunchKernelEx(&cfg, nms_kernel<NT>, a);
+    if (e == cudaErrorNotSupported || e == cudaErrorInvalidValue) {  // a driver without PDL: ordinary launch
+        (void)cudaGetLastError();
+        cfg.numAttrs = 0;
+        e = cudaLaunchKernelEx(&cfg, nms_kernel<NT>, a);
+    }
+    return e;
+}
+
+// threads: 0 / 1024 = the general kernel; 512 = the half-SM one (TRTX_ERR_UNSUPPORTED where it does not cover the call)
+static int nms_launch(NmsArgs& a, int batch, cudaStream_t st, int threads = 0) {
 #ifdef TRTX_NMS_PROBE
     a.dbg = t_nms_stamps;
 #endif
+    TRTX_TL_TAKE(a);
     if (a.pre_topk > kMaxSort) return TRTX_ERR_UNSUPPORTED;
+    if (threads != 0 && threads != kNmsThreads && threads != kNmsThreadsHalf) return TRTX_ERR_UNSUPPORTED;
+    const bool half = threads == kNmsThreadsHalf;
+    if (half && !nms_half_ok(a)) return TRTX_ERR_UNSUPPORTED;
     const size_t smem = nms_smem_bytes(a.pre_topk, a.from_tiles ? a.tiles_per_image : 0);
-    // 227 KB per CTA minus the kernel's static shared memory (histograms, ~18 KB)
-    constexpr size_t kMaxDynSmem = (227 - 20) * 1024;
-    if (smem > kMaxDynSmem) return TRTX_ERR_UNSUPPORTED;
-    // per-device function attribute; cheap and idempotent, so set on every call (no global state)
-    cudaFuncSetAttribute(nms_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxDynSmem);
-    nms_kernel<<<batch, kNmsThreads, smem, st>>>(a);
+    if (smem > (227 - 20) * 1024) return TRTX_ERR_UNSUPPORTED;
+    const cudaError_t e = half ? nms_launch_nt<kNmsThreadsHalf>(a, batch, smem, st) : nms_launch_nt<kNmsThreads>(a, batch, smem, st);
+    if (e != cudaSuccess) {
+        (void)cudaGetLastError();
+        g_last_cuda_error = (int)e;
+        return TRTX_ERR_CUDA;
+    }
     return check_launch();
 }
 
@@ -1007,6 +1073,14 @@ TRTX_API int trtx_probe_set_nms_stamps(void* p) {
     t_nms_stamps = static_cast<long long*>(p);
     return TRTX_OK;
 }
+// probe build only: device buffer of `records` timeline records (common.cuh) for this thread's next launches; null: off
+TRTX_API int trtx_probe_set_timeline(void* p, int records) {
+    t_tl_buf = static_cast<unsigned long long*>(p);
+    t_tl_records = p ? records : 0;
+    t_tl_next = 0;
+    return TRTX_OK;
+}
+TRTX_API size_t trtx_probe_timeline_record_words() { return kTlRecordWords; }
 #endif
 
 TRTX_API size_t trtx_nms_workspace_size(const trtx_nms_params* p, int batch, int max_rows) {
@@ -1096,7 +1170,7 @@ static int yolo_nms_tiles(const trtx_yolo_params* p, const trtx_nms_params* q, i
     a.keep_index = keep_index_dev;
     const int rc = fill_gather(gather, &a.g);
     if (rc) return rc;
-    return nms_launch(a, batch, st);
+    return nms_launch(a, batch, st, p->tune_nms_threads);
 }
 
 TRTX_API int trtx_yolo_decode_nms_enqueue(const trtx_yolo_params* p, const trtx_nms_params* q, int batch,

@@ -32,6 +32,7 @@ struct PreImage {
 struct PreArgs {
     PreImage img[kMaxImagesPerLaunch];
     int dw, dh;
+    TRTX_TL_FIELD  // probe build: this launch's timeline record
 };
 
 // x / 255.0f, correctly rounded, in 3 FP instructions instead of the IEEE division subroutine:
@@ -66,6 +67,7 @@ constexpr int kRowsPerThread = 4;  // 8-row strips measured slower (profiles/r01
 // count is down (no pipe above 60 %), and occupancy is what hides it: 59.4 us at 60 registers, 53.7 at 40, 51.9 at 32.
 template <typename OutT>
 __global__ void __launch_bounds__(256, 8) letterbox_kernel(const __grid_constant__ PreArgs a, OutT* __restrict__ dst) {
+    TRTX_TL(a, kTlLetterbox);
     constexpr int R = kRowsPerThread;
     const int b = blockIdx.z;
     const PreImage& im = a.img[b];
@@ -216,10 +218,12 @@ struct alignas(64) UnitArgs {
     CUtensorMap map[kMaxUnitImages];
     UnitImage img[kMaxUnitImages];
     int dw, dh;
+    TRTX_TL_FIELD  // probe build: this launch's timeline record
 };
 
 template <typename OutT, int WARPS>
 __global__ void __launch_bounds__(WARPS * 32) letterbox_unit_kernel(const __grid_constant__ UnitArgs a, OutT* __restrict__ dst) {
+    TRTX_TL(a, kTlLetterbox);
     constexpr int TW = kUnitTW, TH = WARPS * 8, BOXW = kUnitBoxBytes, ROWS = TH + 1;
     __shared__ __align__(128) uint8_t box[ROWS * BOXW];
     __shared__ uint64_t bar;
@@ -382,6 +386,7 @@ static int launch_unit(const trtx_image_desc* const* d, UnitImage* u, int n, voi
         a.img[i] = u[i];
     }
     dim3 grid((dw + kUnitTW - 1) / kUnitTW, (dh + kUnitWarps * 8 - 1) / (kUnitWarps * 8), n);
+    TRTX_TL_TAKE(a);
     if (out_dtype == TRTX_F32)
         letterbox_unit_kernel<float, kUnitWarps><<<grid, kUnitWarps * 32, 0, st>>>(a, static_cast<float*>(dst));
     else
@@ -605,6 +610,7 @@ TRTX_API int trtx_preprocess_batch_enqueue(const trtx_image_desc* images_host, i
         constexpr int R = kRowsPerThread;
         dim3 block(128, 2, 1);  // 128 columns x (2 x R) rows per block
         dim3 grid((dst_w + 127) / 128, (dst_h + 2 * R - 1) / (2 * R), ng);
+        TRTX_TL_TAKE(g);
         if (out_dtype == TRTX_F32)
             letterbox_kernel<float><<<grid, block, 0, st>>>(g, static_cast<float*>(dst_dev));
         else

@@ -162,6 +162,7 @@ __device__ __forceinline__ void scan_classes_h8(const __half* __restrict__ row0,
 // --------------------------------------------------------------------------------------------
 template <typename T, int VEC, int SLICES, int U>
 __global__ void __launch_bounds__(32 * SLICES) yolo_v8_scan_kernel(const __grid_constant__ YoloArgs a) {
+    TRTX_TL(a, kTlScan);
     constexpr int TILE = 32 * VEC;
     __shared__ float s_m[SLICES > 1 ? SLICES - 1 : 1][TILE];   // per class slice: max logit,
     __shared__ float s_m2[SLICES > 1 ? SLICES - 1 : 1][TILE];  // max logit before its class,
@@ -232,6 +233,10 @@ __global__ void __launch_bounds__(32 * SLICES) yolo_v8_scan_kernel(const __grid_
         else
             scan_classes<T, VEC, U>(base + (size_t)(4 + c0) * g + a0, g, c1 - c0, c0, s);
     }
+    // The streaming loop is done: let a kernel launched programmatically behind this one (nms_kernel) get its CTAs placed
+    // during the candidate epilogue below.  It reads nothing before its griddepcontrol.wait, which waits for this grid
+    // to complete, so where this trigger sits only moves time, never results.
+    asm volatile("griddepcontrol.launch_dependents;");
 
     if constexpr (SLICES > 1) {
         bool mine = false;
@@ -836,7 +841,9 @@ static int launch_v8(const YoloArgs& a, const YoloLayout& L, int grid, cudaStrea
     return TRTX_ERR_UNSUPPORTED;  // (slices, rows in flight) pair that is not built
 }
 
-int yolo_scan_launch(const YoloArgs& a, const YoloLayout& L, int in_dtype, int batch, cudaStream_t st) {
+int yolo_scan_launch(const YoloArgs& a_in, const YoloLayout& L, int in_dtype, int batch, cudaStream_t st) {
+    YoloArgs a = a_in;
+    TRTX_TL_TAKE(a);
     const int grid = batch * L.tiles_per_image;
     if (L.pipe) {
         const int rc = yolo_scan_pipe_launch(a, L, in_dtype, batch, st);

@@ -47,6 +47,7 @@ struct YoloArgs {
     int prefetch_box;  // register scan: L2-prefetch the 4 box rows while the class rows stream
     int* tile_count;
     float4* cand;
+    TRTX_TL_FIELD  // probe build: this launch's timeline record
 };
 
 struct YoloLayout {

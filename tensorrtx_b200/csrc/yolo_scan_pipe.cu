@@ -66,6 +66,7 @@ template <typename T>
 __global__ void __launch_bounds__(1024, 1)
         yolo_v8_scan_pipe_kernel(const __grid_constant__ YoloArgs a, const __grid_constant__ TmaMaps maps,
                                  const __grid_constant__ PipeGeom geo, int total_stiles, int stages, int stage_bytes) {
+    TRTX_TL(a, kTlScan);
     extern __shared__ __align__(128) unsigned char smem[];
     unsigned char* stage_base = smem;
     uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + (size_t)stages * stage_bytes);
@@ -100,6 +101,7 @@ __global__ void __launch_bounds__(1024, 1)
                     tma_load_3d(dst + (size_t)ch * kTileAnchors * sizeof(T), &maps.m[l], col0, ch, b, &full_bar[s]);
             }
         }
+        asm volatile("griddepcontrol.launch_dependents;");  // every load is issued (see yolo_v8_scan_kernel)
         return;
     }
 
@@ -167,6 +169,7 @@ __global__ void __launch_bounds__(1024, 1)
         __syncwarp();
         if (lane == 0) mbar_arrive(&empty_bar[s]);  // one of the releases the producer waits for
     }
+    asm volatile("griddepcontrol.launch_dependents;");
 }
 
 

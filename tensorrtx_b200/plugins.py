@@ -43,11 +43,12 @@ def _stream(stream=None) -> int:
     return int(stream)
 
 
-def _tune(params, slices: int = 0, rows: int = 0, tma: int = 0, stages: int = 0, box: int = 0) -> None:
-    """Per-plugin launch tuning of the scan kernel (trtx_yolo_params.tune_*; 0 = default).  Plain data inside the
-    plugin's own parameter block -- nothing global, clones / other plugins are unaffected."""
+def _tune(params, slices: int = 0, rows: int = 0, tma: int = 0, stages: int = 0, box: int = 0, nms_threads: int = 0) -> None:
+    """Per-plugin launch tuning of the scan kernel and of the fused NMS (trtx_yolo_params.tune_*; 0 = default).  Plain
+    data inside the plugin's own parameter block -- nothing global, clones / other plugins are unaffected."""
     params.tune_class_slices, params.tune_rows_in_flight = int(slices), int(rows)
     params.tune_tma_pipeline, params.tune_tma_stages, params.tune_box_prefetch = int(tma), int(stages), int(box)
+    params.tune_nms_threads = int(nms_threads)
 
 
 def float_le_threshold(x: float) -> float:

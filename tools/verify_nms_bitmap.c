@@ -3,6 +3,9 @@
 // (32 rows per chunk, suppression by kept rows of earlier chunks through the `kept` words, one "ballot" per kept row
 // found with ffs) -- against plain greedy NMS on the same overlap relation.  The overlap relation is random with a
 // tunable density (clusters), so every segment length and chunk boundary (31/32/33, 63/64/65, 95/96) is hit.
+// Both block sizes of nms_kernel (1024 and 512 threads) are replayed: the unit list is walked with the kernel's thread
+// stride (every unit exactly once), and the same segment is also resolved by the long-segment path (whole CTA, chunks of
+// 32: tests against the kept rows with stride NT, chunk member i on warp i mod NT/32, warp 0's serial resolve).
 // usage: verify_nms_bitmap [segments_per_thread]
 #include <omp.h>
 #include <stdint.h>
@@ -68,9 +71,15 @@ int main(int argc, char** argv) {
                     }
                 }
             for (int u = 0; u < U; ++u) layout_ok &= seen[u];
-            // (1b) one byte of the row's bitmap per unit
+            for (int nt_i = 0; nt_i < 2; ++nt_i) {
+            const int NT = nt_i == 0 ? 1024 : 512, NW = NT / 32;
+            // (1b) one byte of the row's bitmap per unit; thread tid takes units tid, tid + NT, ...
             unsigned char mask_bytes[KSHORT][12];
             memset(mask_bytes, 0, sizeof(mask_bytes));
+            memset(seen, 0, (size_t)(U > 0 ? U : 1));
+            for (int tid = 0; tid < NT; ++tid)
+                for (int u = tid; u < U; u += NT) seen[u]++;
+            for (int u = 0; u < U; ++u) layout_ok &= seen[u] == 1;
             for (int u = 0; u < U && layout_ok; ++u) {
                 const int li = unit_row[u], g = unit_g[u];
                 unsigned bits = 0;
@@ -109,10 +118,47 @@ int main(int argc, char** argv) {
                 for (int lane = 0; lane < 32; ++lane)
                     if ((alive >> lane) & 1u) keep[c * 32 + lane] = 1;
             }
+            // (3) the long-segment path on the same segment: chunks of 32 rows against the kept rows so far
+            unsigned char keep_long[KSHORT];
+            memset(keep_long, 0, sizeof(keep_long));
+            int krow[KSHORT], n_kept = 0, members_ok = 1;
+            for (int c0 = 0; c0 < m; c0 += 32) {
+                const int nchunk = m - c0 < 32 ? m - c0 : 32;
+                unsigned rem_bits = 0, sup[32];
+                for (int tid = 0; tid < NT; ++tid)
+                    for (int p = tid; p < 32 * n_kept; p += NT) {
+                        const int i = p & 31, k = p >> 5;
+                        if (i < nchunk && ov[krow[k]][c0 + i]) rem_bits |= 1u << i;
+                    }
+                int written[32] = {0};
+                for (int warp = 0; warp < NW; ++warp)
+                    for (int i = warp; i < 32; i += NW) {
+                        unsigned mm = 0;
+                        for (int lane = 0; lane < 32; ++lane)
+                            if (i < nchunk && lane < i && ov[c0 + lane][c0 + i]) mm |= 1u << lane;  // __ballot_sync
+                        sup[i] = mm;
+                        written[i]++;
+                    }
+                for (int i = 0; i < 32; ++i) members_ok &= written[i] == 1;
+                unsigned alive = ~rem_bits & (nchunk == 32 ? 0xffffffffu : ((1u << nchunk) - 1u));
+                for (unsigned rem = alive; rem != 0u;) {
+                    const int jx = __builtin_ffs((int)rem) - 1;
+                    unsigned kill = 0;
+                    for (int lane = 0; lane < 32; ++lane) kill |= ((sup[lane] >> jx) & 1u) << lane;
+                    alive &= ~kill;
+                    rem = alive & ~((2u << jx) - 1u);
+                }
+                for (int lane = 0; lane < 32; ++lane)
+                    if ((alive >> lane) & 1u) {
+                        keep_long[c0 + lane] = 1;
+                        krow[n_kept++] = c0 + lane;
+                    }
+            }
             ++total;
-            if (!layout_ok || memcmp(keep, keep_ref, (size_t)m) != 0) {
+            if (!layout_ok || !members_ok || memcmp(keep, keep_ref, (size_t)m) != 0 || memcmp(keep_long, keep_ref, (size_t)m) != 0) {
                 ++bad;
-                if (bad < 5) printf("MISMATCH m=%d dens=%u layout_ok=%d\n", m, dens, layout_ok);
+                if (bad < 5) printf("MISMATCH NT=%d m=%d dens=%u layout_ok=%d members_ok=%d\n", NT, m, dens, layout_ok, members_ok);
+            }
             }
         }
     }
