@@ -49,7 +49,7 @@ TRTX_API const char* trtx_version(void);
 TRTX_API int trtx_last_cuda_error(void);
 /* sizeof() of the parameter structs as THIS library was compiled, so that an FFI binding (ctypes, cgo, ...) can check its
  * mirror of the layout: which = 0 trtx_yolo_params, 1 trtx_nms_params, 2 trtx_retina_params, 3 trtx_image_desc,
- * 4 trtx_mask_params; anything else 0. */
+ * 4 trtx_mask_params, 5 trtx_refinedet_params; anything else 0. */
 TRTX_API size_t trtx_abi_sizeof(int which);
 
 /* =====================================================================================
@@ -409,6 +409,55 @@ typedef struct trtx_mask_params {
  * masks_dev: [batch, max_masks, net_h, net_w] fp32; slots >= count are left untouched.  One launch. */
 TRTX_API int trtx_process_mask_enqueue(const trtx_mask_params* p, int batch, const float* proto_dev, const float* dets_dev,
                                        int max_rows, float* masks_dev, trtx_stream_t stream);
+
+/* =====================================================================================
+ * 7. RefineDet post-process -- two-stage prior decode + per-class greedy NMS
+ *    replaces PriorBox / decode / nms and the driver glue of refinedet/refinedet.cpp:553-790, which the
+ *    reference writes with tensor-library ops in fp64 for batch 1 (host loop over classes, ~20 launches and
+ *    4 device-to-host syncs per kept box).  Every image of the batch, three launches, no sync.
+ *    Inputs per image, row-major per prior, soft-maxed by the network (refinedet.cpp:267-290, :488-506):
+ *      arm_loc [P,4], arm_conf [P,2], odm_loc [P,4], odm_conf [P,C]  (class 0 = background), fp32.
+ *    Arithmetic (all fp64, every operation rounded on its own like the eager reference):
+ *      ARM box  = (p_xy + (loc_xy*v0)*p_wh, p_wh*exp(loc_wh*v1))           (decode, :600-616)
+ *      ODM box  = decode(odm_loc, ARM box) as corners c3 = xy - wh/2, c4 = c3 + wh
+ *      candidate of class c >= 1: arm_conf[p][1] > obj_thresh && odm_conf[p][c] > conf_thresh (:738-760)
+ *      per class: the top_k highest scores, greedy NMS suppressing !(IoU < nms_thresh) with the suppressor's
+ *      corners rounded to fp32 inside the clamps (nms(), :632-695).
+ *    Equal scores rank the lower prior index first (also at the top_k cut); the reference's sort is unstable there.
+ *    output_dev: [batch, 1 + max_out*7] fp32 = count, rows (x1, y1, x2, y2, score, label, keep = 1), classes
+ *    ascending, rows of a class in keep order (score descending); count = min(total kept, max_out); floats past
+ *    the last row are zero.
+ * ===================================================================================== */
+#define TRTX_REFINEDET_MAX_TOPK 1024   /* candidates per (image, class) entering the greedy NMS */
+#define TRTX_REFINEDET_MAX_CLASSES 91  /* including the background class */
+typedef struct trtx_refinedet_params {
+    int32_t num_priors;  /* P: rows of every input (6375 for the 320 model, :731) */
+    int32_t num_classes; /* C including background (25, :756) */
+    float obj_thresh;    /* ARM objectness gate, 0.01 (obj_threshed, :738) */
+    float conf_thresh;   /* ODM class gate, 0.01 (mask_thresh, :753) */
+    float nms_thresh;    /* 0.45 (overlap, :765) */
+    int32_t top_k;       /* 1000 (:766), 1 .. TRTX_REFINEDET_MAX_TOPK */
+    int32_t max_out;     /* output rows per image */
+    float variance[2];   /* 0.1, 0.2 (:602) */
+    int32_t reserved;    /* 0 */
+} trtx_refinedet_params;
+
+/* The prior table (PriorBox, :553-597) as a HOST function: per level k, per cell (i, j) of the f_k x f_k map, 3 boxes
+ * (cx, cy, s, s), (cx, cy, s*sqrt(ar), s/sqrt(ar)), (cx, cy, s/sqrt(ar), s*sqrt(ar)), clamped to [0, 1], with the
+ * reference's float/double rounding.  Returns P = 3 * sum f_k^2 (0 on invalid arguments); writes P*4 floats to out_host
+ * unless it is NULL. */
+TRTX_API int trtx_refinedet_priors(int image_size, int num_levels, const int* feature_maps, const int* steps,
+                                   const int* min_sizes, const float* aspect_ratios, float* out_host);
+TRTX_API size_t trtx_refinedet_workspace_size(const trtx_refinedet_params* p, int batch);
+/* priors_dev: [P,4] fp32 (trtx_refinedet_priors).  Error codes: TRTX_ERR_INVALID for null pointers, priors / loc
+ * pointers not 16-byte aligned or arm_conf not 8-byte aligned, batch < 1,
+ * num_classes < 2, top_k outside 1 .. TRTX_REFINEDET_MAX_TOPK, max_out < 1; TRTX_ERR_UNSUPPORTED for
+ * num_classes > TRTX_REFINEDET_MAX_CLASSES or a prior count whose candidate list does not fit on chip;
+ * TRTX_ERR_WORKSPACE when workspace_bytes < trtx_refinedet_workspace_size. */
+TRTX_API int trtx_refinedet_detect_enqueue(const trtx_refinedet_params* p, int batch, const float* priors_dev,
+                                           const float* arm_loc_dev, const float* arm_conf_dev, const float* odm_loc_dev,
+                                           const float* odm_conf_dev, float* output_dev, void* workspace_dev,
+                                           size_t workspace_bytes, trtx_stream_t stream);
 
 #ifdef __cplusplus
 }

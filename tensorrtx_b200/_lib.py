@@ -94,6 +94,23 @@ class MaskParams(C.Structure):
                                          "coeff_offset", "max_masks")]
 
 
+class RefineDetParams(C.Structure):
+    _fields_ = [
+        ("num_priors", C.c_int32),
+        ("num_classes", C.c_int32),
+        ("obj_thresh", C.c_float),
+        ("conf_thresh", C.c_float),
+        ("nms_thresh", C.c_float),
+        ("top_k", C.c_int32),
+        ("max_out", C.c_int32),
+        ("variance", C.c_float * 2),
+        ("reserved", C.c_int32),
+    ]
+
+
+REFINEDET_MAX_TOPK = 1024
+REFINEDET_MAX_CLASSES = 91
+
 # TRTX_LIB: another build of the same ABI (the probe build of tools/nms_probe.py); default = the in-tree release library
 LIB_PATH = Path(os.environ.get("TRTX_LIB") or Path(__file__).resolve().parent / "lib" / "libtrtx_hot.so")
 
@@ -144,6 +161,10 @@ SYMBOLS = {
     "trtx_peer_open": (_i, [C.POINTER(C.c_ubyte), C.POINTER(C.c_void_p)]),
     "trtx_peer_close": (_i, [_vp]),
     "trtx_peer_free": (_i, [_vp]),
+    "trtx_refinedet_priors": (_i, [_i, _i, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int),
+                                   C.POINTER(C.c_float), _vp]),
+    "trtx_refinedet_workspace_size": (_sz, [C.POINTER(RefineDetParams), _i]),
+    "trtx_refinedet_detect_enqueue": (_i, [C.POINTER(RefineDetParams), _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
 }
 
 _lib = None
@@ -164,7 +185,7 @@ def load() -> C.CDLL:
         fn = getattr(lib, name)  # AttributeError if the library does not export a declared symbol
         fn.restype = res
         fn.argtypes = args
-    for which, st in enumerate((YoloParams, NmsParams, RetinaParams, ImageDesc, MaskParams)):
+    for which, st in enumerate((YoloParams, NmsParams, RetinaParams, ImageDesc, MaskParams, RefineDetParams)):
         if lib.trtx_abi_sizeof(which) != C.sizeof(st):
             raise TrtxError(f"{LIB_PATH} was built from a different trtx_hot.h: sizeof({st.__name__}) = "
                             f"{lib.trtx_abi_sizeof(which)} in the library, {C.sizeof(st)} in the binding (rebuild)")

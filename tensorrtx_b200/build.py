@@ -18,7 +18,7 @@ CSRC = PKG / "csrc"
 LIBDIR = PKG / "lib"
 LIB = LIBDIR / "libtrtx_hot.so"
 
-SOURCES = ["yolo_decode.cu", "yolo_scan_pipe.cu", "nms.cu", "retina_decode.cu", "rcnn.cu", "preprocess.cu", "mask.cu", "roi_align.cu", "calib_host.cu"]
+SOURCES = ["yolo_decode.cu", "yolo_scan_pipe.cu", "nms.cu", "retina_decode.cu", "rcnn.cu", "preprocess.cu", "mask.cu", "roi_align.cu", "calib_host.cu", "refinedet.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
@@ -91,9 +91,11 @@ def build(force: bool = False, verbose: bool = False, probe: bool = False, defin
 
 def build_oracle() -> Path:
     """Compile the CPU oracle (test infrastructure) and, when /root/reference exists, oracle/_ref."""
-    r = subprocess.run(["make", "-C", str(ROOT / "oracle")], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
-    if r.returncode != 0:
-        raise RuntimeError(f"oracle build failed:\n{r.stdout}")
+    for extra in ([], ["-f", "refinedet.mk"]):
+        r = subprocess.run(["make", "-C", str(ROOT / "oracle"), *extra], stdout=subprocess.PIPE, stderr=subprocess.STDOUT,
+                           text=True)
+        if r.returncode != 0:
+            raise RuntimeError(f"oracle build failed:\n{r.stdout}")
     return ROOT / "oracle" / "libtrtx_oracle.so"
 
 

@@ -898,6 +898,7 @@ TRTX_API size_t trtx_abi_sizeof(int which) {
         case 2: return sizeof(trtx_retina_params);
         case 3: return sizeof(trtx_image_desc);
         case 4: return sizeof(trtx_mask_params);
+        case 5: return sizeof(trtx_refinedet_params);
         default: return 0;
     }
 }

@@ -8,6 +8,7 @@ like the reference's call sites:
   YoloPluginCreator      yolov8/plugin/yololayer.h:87-109    (field "combinedInfo", block.cpp:264-296)
   DecodePlugin           retinaface/decode.h:22-83           ("Decode_TRT" v1)
   RpnDecodePlugin / RpnNmsPlugin / PredictorDecodePlugin / BatchedNmsPlugin   rcnn/*Plugin.h
+  RefineDetPostprocess   refinedet/refinedet.cpp:553-790     (PriorBox + decode + per-class nms of doInference)
   batch_nms / cuda_decode+cuda_nms / cuda_batch_preprocess   yolov8/include/postprocess.h, preprocess.h
 
 All compute goes through the C ABI of libtrtx_hot.so (include/trtx_hot.h); torch is used only for
@@ -993,3 +994,80 @@ def letterbox_matrix(src_w: int, src_h: int, dst_w: int, dst_h: int):
     m = (C.c_float * 6)()
     L.load().trtx_letterbox_matrix(src_w, src_h, dst_w, dst_h, m)
     return list(m)
+
+
+# --------------------------------------------------------------------------------------------------
+# RefineDet post-process (refinedet/refinedet.cpp:553-790): PriorBox + two-stage decode + per-class NMS
+# --------------------------------------------------------------------------------------------------
+def refinedet_priors(image_size: int = 320, feature_maps=(40, 20, 10, 5), steps=(8, 16, 32, 64),
+                     min_sizes=(32, 64, 128, 256), aspect_ratios=(2, 2, 2, 2)):
+    """PriorBox() of refinedet.cpp:553-597 -> float32 [P, 4] (cx, cy, w, h), computed on the host by the library."""
+    import numpy as np
+
+    lib = L.load()
+    n = len(feature_maps)
+    if not (len(steps) == len(min_sizes) == len(aspect_ratios) == n):
+        raise L.TrtxError("feature_maps, steps, min_sizes and aspect_ratios need one entry per level")
+    args = (int(image_size), n, (C.c_int * n)(*map(int, feature_maps)), (C.c_int * n)(*map(int, steps)),
+            (C.c_int * n)(*map(int, min_sizes)), (C.c_float * n)(*map(float, aspect_ratios)))
+    P = lib.trtx_refinedet_priors(*args, None)
+    if P <= 0:
+        raise L.TrtxError("trtx_refinedet_priors: invalid prior geometry")
+    out = np.empty((P, 4), np.float32)
+    lib.trtx_refinedet_priors(*args, out.ctypes.data)
+    return out
+
+
+class RefineDetPostprocess:
+    """The post-process of RefineDet's doInference (refinedet.cpp:729-790) for a whole batch: the four engine outputs
+    arm_loc [B,P,4], arm_conf [B,P,2], odm_loc [B,P,4], odm_conf [B,P,C] (fp32 device tensors, soft-maxed by the
+    network) -> [B, 1 + max_out*7] fp32 = count, rows (x1, y1, x2, y2, score, label, 1) with classes ascending and the
+    rows of a class in keep order.  Defaults are the reference's 320 model.  The prior table is built and uploaded
+    once; enqueue() is three kernel launches and no synchronisation."""
+
+    def __init__(self, image_size: int = 320, feature_maps=(40, 20, 10, 5), steps=(8, 16, 32, 64),
+                 min_sizes=(32, 64, 128, 256), aspect_ratios=(2, 2, 2, 2), num_classes: int = 25,
+                 obj_thresh: float = 0.01, conf_thresh: float = 0.01, nms_thresh: float = 0.45, top_k: int = 1000,
+                 max_out: int | None = None, variance=(0.1, 0.2), device=None):
+        self._lib = L.load()
+        self.priors_host = refinedet_priors(image_size, feature_maps, steps, min_sizes, aspect_ratios)
+        self.device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+        self.priors = torch.from_numpy(self.priors_host).to(self.device)
+        p = L.RefineDetParams()
+        p.num_priors, p.num_classes = self.priors_host.shape[0], int(num_classes)
+        p.obj_thresh, p.conf_thresh, p.nms_thresh = float(obj_thresh), float(conf_thresh), float(nms_thresh)
+        p.top_k = int(top_k)
+        # the reference keeps every row: up to top_k per foreground class
+        p.max_out = int(max_out) if max_out is not None else (int(num_classes) - 1) * int(top_k)
+        p.variance[0], p.variance[1] = float(variance[0]), float(variance[1])
+        self.params = p
+        self._ws = None
+
+    @property
+    def num_priors(self) -> int:
+        return self.params.num_priors
+
+    def output_elems(self) -> int:
+        return 1 + self.params.max_out * 7
+
+    def getWorkspaceSize(self, batch: int) -> int:
+        return int(self._lib.trtx_refinedet_workspace_size(C.byref(self.params), int(batch)))
+
+    def enqueue(self, arm_loc, arm_conf, odm_loc, odm_conf, out=None, workspace=None, stream=None) -> torch.Tensor:
+        batch = int(arm_loc.shape[0])
+        P, Cn = self.params.num_priors, self.params.num_classes
+        for t, w in ((arm_loc, 4), (arm_conf, 2), (odm_loc, 4), (odm_conf, Cn)):
+            if tuple(t.shape) != (batch, P, w) or t.dtype != torch.float32:
+                raise L.TrtxError(f"expected float32 [{batch}, {P}, {w}], got {t.dtype} {tuple(t.shape)}")
+        if out is None:
+            out = torch.empty((batch, self.output_elems()), dtype=torch.float32, device=arm_loc.device)
+        if workspace is None:
+            need = self.getWorkspaceSize(batch)
+            if self._ws is None or self._ws.numel() < need:
+                self._ws = torch.empty(need, dtype=torch.uint8, device=arm_loc.device)
+            workspace = self._ws
+        L.check(self._lib.trtx_refinedet_detect_enqueue(
+            C.byref(self.params), batch, _ptr(self.priors), _ptr(arm_loc), _ptr(arm_conf), _ptr(odm_loc),
+            _ptr(odm_conf), _ptr(out), _ptr(workspace), workspace.numel() * workspace.element_size(),
+            _stream(stream)), "trtx_refinedet_detect_enqueue")
+        return out

@@ -218,3 +218,74 @@ def predictor_inputs(batch: int, seed: int = 0, N: int = 1000, Ccls: int = 80, i
     h = rng.uniform(16, image_h * 0.3, (batch, N)).astype(np.float32)
     props = np.stack([x1, y1, np.minimum(x1 + w, image_w), np.minimum(y1 + h, image_h)], -1).astype(np.float32)
     return scores, deltas, props
+
+
+def _softmax(x):
+    e = np.exp(x - x.max(-1, keepdims=True))
+    return (e / e.sum(-1, keepdims=True)).astype(np.float32)
+
+
+def _untie(conf):
+    """Nudge equal values of every (image, class) column of [B, P, C] up by ulps until the column has no ties."""
+    for b in range(conf.shape[0]):
+        for c in range(conf.shape[2]):
+            col = conf[b, :, c]
+            while True:
+                order = np.argsort(col, kind="stable")
+                s = col[order]
+                dup = np.nonzero(s[1:] == s[:-1])[0] + 1
+                if dup.size == 0:
+                    break
+                col[order[dup]] = np.nextafter(s[dup], np.float32(np.inf))
+    return conf
+
+
+REFINEDET_SUITES = ("default", "dense", "gated_off", "ties", "overflow")
+
+
+def refinedet_heads(batch: int, seed: int = 0, num_priors: int = 6375, num_classes: int = 25, n_obj: int = 24,
+                    suite: str = "default"):
+    """RefineDet engine outputs (refinedet.cpp:733-736), soft-maxed like the network: -> (arm_loc [B,P,4],
+    arm_conf [B,P,2], odm_loc [B,P,4], odm_conf [B,P,C]) float32.  Background-dominant: ~18 % of priors pass the
+    objectness gate and ~5 % of those are candidates of a given class; per image `n_obj` planted objects (a run of 9
+    consecutive priors -- 3 cells of the same map row -- with a confident class and small regressions, so that they
+    overlap).  Suites: "dense" gives class 1 of every image ~2000 candidates (the top_k = 1000 select runs), "gated_off"
+    puts every objectness below the gate, "ties" rounds all scores to multiples of 1/256, "overflow" sets ~2 % of the
+    size regressions to +-4000 (exp overflows to inf / underflows to 0, corners become inf or NaN).  Every suite except
+    "ties" is tie-free within each (image, class) column."""
+    if suite not in REFINEDET_SUITES:
+        raise ValueError(suite)
+    rng = _rng(seed)
+    B, P, C = batch, num_priors, num_classes
+    arm_loc = rng.normal(0, 0.5, (B, P, 4)).astype(np.float32)
+    odm_loc = rng.normal(0, 0.5, (B, P, 4)).astype(np.float32)
+    arm_logit = np.stack([np.zeros((B, P)), rng.normal(-6.0, 1.5, (B, P))], -1)
+    odm_logit = rng.normal(0.0, 1.0, (B, P, C))
+    odm_logit[..., 0] += 6.0
+    for b in range(B):
+        for _ in range(n_obj):
+            p0 = int(rng.integers(0, P - 9))
+            c = int(rng.integers(1, C))
+            sl = slice(p0, p0 + 9)
+            arm_logit[b, sl, 1] = rng.normal(3.0, 1.0, 9)
+            odm_logit[b, sl, c] += rng.normal(9.0, 1.0, 9)
+            arm_loc[b, sl] = rng.normal(0, 0.2, (9, 4))
+            odm_loc[b, sl] = rng.normal(0, 0.2, (9, 4))
+    if suite == "dense":
+        for b in range(B):
+            sel = rng.choice(P, 2000, replace=False)
+            arm_logit[b, sel, 1] = rng.normal(3.0, 1.0, sel.size)
+            odm_logit[b, sel, 1] += rng.normal(7.0, 1.0, sel.size)
+    arm_conf = _softmax(arm_logit)
+    if suite == "gated_off":
+        arm_conf[..., 1] = np.minimum(arm_conf[..., 1], np.float32(0.005))
+    odm_conf = _softmax(odm_logit)
+    if suite == "ties":
+        odm_conf = (np.round(odm_conf * 256) / 256).astype(np.float32)
+    else:
+        odm_conf = _untie(odm_conf)
+    if suite == "overflow":
+        for loc in (arm_loc, odm_loc):
+            m = rng.random((B, P, 2)) < 0.02
+            loc[..., 2:][m] = np.where(rng.random(int(m.sum())) < 0.5, 4000.0, -4000.0).astype(np.float32)
+    return arm_loc, arm_conf, odm_loc, odm_conf
